@@ -3,6 +3,10 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
                     [--optimizer none|lamb|adamw] [--no-overlap] [--drop-path P] [--no-graph] [--no-cpu-baseline]
+                    [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step handed its caller as DIR/<name>.npy (see dump_outputs); the inputs
+and the initial weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 Metric (BASELINE.json): hybrid octic ViT-H/14 (DeiT-III: embed 1280, depth 32, heads 16, patch 14, 224 px) images/s,
 forward + backward (+ NCCL gradient all-reduce when N > 1), bf16 compute / fp32 residual, synthetic images, random-init
@@ -217,6 +221,48 @@ def run_reference_arm(args):
 
 
 # ----------------------------------------------------------------------------------------------------------------
+# outputs of the timed step, for comparing two builds
+# ----------------------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 22          # positions drawn per sample: at most 16 MB per array in fp32, ~33 MB in all
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir: str, loss: torch.Tensor, fg, updated_params: bool) -> None:
+    """Writes the step's results as float32 / float64 .npy files:
+        loss.npy          the loss, float32 [1]
+        grad_norm.npy     L2 norm of every trainable parameter's gradient, float64, in model.parameters() order
+        grad_sample.npy   the gradient at fixed positions over all trainable elements, float32, in position order:
+                          DUMP_SAMPLE draws with seed DUMP_SEED, repeats removed (4,169,746 distinct positions for the
+                          headline model)
+    and, when the step also ran the optimizer, param_norm.npy / param_sample.npy: the updated parameters, same layout.
+    The full gradient (1.4 GB for the headline model) is too large to keep; the per-parameter norms catch an error in
+    any one tensor, the sample compares element by element.  The weight-gradient kernels reduce with atomic adds, so
+    two runs of the same build differ in the last bits; profiles/r03_bench_dump_spread.txt records how much."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    params = fg.params
+    numels = torch.tensor([p.numel() for p in params])
+    ends = numels.cumsum(0)
+    pick = torch.randint(int(ends[-1]), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(DUMP_SEED)).unique()
+    owner = torch.searchsorted(ends, pick, right=True)
+    local = pick - (ends - numels)[owner]
+    bounds = torch.searchsorted(owner, torch.arange(len(params) + 1)).tolist()
+
+    def sample_and_norms(tensors):
+        vals = [t.detach().reshape(-1)[local[bounds[i]:bounds[i + 1]].to(t.device)] for i, t in enumerate(tensors)]
+        norms = [torch.linalg.vector_norm(t.detach(), dtype=torch.float64) for t in tensors]
+        return torch.cat(vals).float().cpu().numpy(), torch.stack(norms).cpu().numpy()
+
+    arrays = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    arrays["grad_sample"], arrays["grad_norm"] = sample_and_norms([p.grad for p in params])
+    if updated_params:
+        arrays["param_sample"], arrays["param_norm"] = sample_and_norms(params)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
+# ----------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------
 def run_ours(args):
@@ -301,8 +347,15 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_dev = timed(lambda: step(img_dev, tgt_dev), args.steps)
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(img_dev, tgt_dev)
+    ms_dev = timed(timed_step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the untimed eager steps below overwrite the gradients (and, with an optimizer, the parameters)
+        dump_outputs(args.dump_outputs, last["loss"], fg, updated_params=opt is not None)
     # launches of our kernels inside the timed region: counted on one eager step (a graph replay launches the same nodes)
     from octic_vits_b200 import functional as OF
     if gstep.graphed:
@@ -435,7 +488,13 @@ def main():
                          "from inside the captured graph while the octic half is still in backward (DESIGN.md section 5)")
     ap.add_argument("--optimizer", default="none", choices=["none", "lamb", "adamw"],
                     help="also run the fused parameter update every step (the headline metric is fwd+bwd)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the (sampled) gradients of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
