@@ -61,7 +61,7 @@ int octic_device_ok(void);
  * zero-padded to a multiple of 64; a group picks B0 or B1 with b_map.
  * --------------------------------------------------------------------------------------------------------- */
 typedef struct {
-  int a_col;    /* first column of A used by this group                     */
+  int a_col;    /* first column of A used by this group (multiple of 8)     */
   int k;        /* contraction length (<= padded weight columns)            */
   int b_map;    /* 0 -> b0, 1 -> b1                                         */
   int b_row;    /* first weight row of this group                           */
@@ -85,7 +85,7 @@ typedef struct {
   float* resid_out; long ldr; /* EPI_RESID destination (may alias resid_in)                            */
   const float* row_scale;     /* EPI_RESID: per-sample scale (DropPath keep-mask / keep_prob), or NULL */
   int rows_per_sample;
-  void* branch_out; long ldb; /* optional bf16 copy of acc + bias                                      */
+  void* branch_out; long ldb; /* optional bf16 copy of acc + bias (EPI_GELU_BF16: row stride ldo; ldb 0 or ldo) */
   int remap_group; int remap_extra; int remap_off; /* EPI_RESID/EPI_F32 row remap: m' = m + (m/remap_group)*remap_extra + remap_off (0 = identity) */
   /* EPI_BF16 head remap (0 heads = off).  Feature n of a group with n_g outputs is read as [S][H][c_g]
    * (c_g = n_g / (S*H), even) and stored at column s*head_D + h*(head_D/H) + head_off[group] + j instead of
@@ -102,7 +102,7 @@ int octic_gemm_bf16(const octic_gemm_desc* desc, void* stream);
  * (the caller zeroes or pre-loads dW).  Replaces the autograd wgrad of nn.Linear inside LinearD8
  * (octic_vits/d8_layers.py:117-127). */
 typedef struct {
-  int dy_col; int x_col; int n_out; int k_in;
+  int dy_col; int x_col; int n_out; int k_in;   /* dy_col, x_col: multiples of 8 */
   float* dw; long ldw;
 } octic_wgrad_group;
 
@@ -117,6 +117,34 @@ typedef struct {
 } octic_wgrad_desc;
 
 int octic_gemm_wgrad_bf16(const octic_wgrad_desc* desc, void* stream);
+
+/* Launch plan of the last GEMM this host thread launched (octic_gemm_bf16, octic_gemm_wgrad_bf16 or a wrapper over them:
+ * LinearD8 forward / dgrad / wgrad, the dense helpers).  It is recorded from the same values the launch uses, right
+ * before the kernel is launched, so a test can assert which code path a shape takes.  Returns OCTIC_ERR_ARG when this
+ * thread has launched no GEMM yet.  A refused call (a negative return before the launch) leaves the previous plan. */
+#define OCTIC_GEMM_PLAN_TN 0
+#define OCTIC_GEMM_PLAN_WGRAD 1
+typedef struct {
+  int kind;          /* OCTIC_GEMM_PLAN_TN or OCTIC_GEMM_PLAN_WGRAD                                              */
+  int mode;          /* tn: OCTIC_EPI_*; wgrad: -1                                                                 */
+  int ncta;          /* 1 = single CTAs, 2 = CTA pairs (cta_group::2, 256-row tiles)                              */
+  int num_stages;    /* TMA ring depth                                                                            */
+  int ws;            /* tn: weight-stationary tile order                                                          */
+  int block_n;       /* N tile (tn: output columns; wgrad: X columns)                                              */
+  int grid;          /* CTAs launched (pairs count twice)                                                          */
+  int num_m_blocks;  /* tn: blocks of 128 * ncta rows                                                              */
+  int total_tiles;   /* output tiles of the launch                                                                */
+  int kb_total;      /* wgrad: 64-token k-blocks                                                                  */
+  int full_rounds;   /* wgrad: rounds in which every CTA (pair) takes one whole tile                               */
+  int rem_tiles;     /* wgrad: tiles left after the full rounds                                                    */
+  int rem_splits;    /* wgrad: > 0 = each remaining tile cut into this many token ranges; 0 = one stream-K line     */
+  int splits;        /* wgrad: the descriptor's splits                                                             */
+  int packed;        /* tn: 1 = bf16-packed epilogue staging where it applies (OCTIC_GEMM_PACKED unset)            */
+  int direct;        /* tn: 1 = register-direct epilogue for this launch's mode (OCTIC_GEMM_DIRECT mask)           */
+  int roles_low;     /* 1 = TMA producer / MMA issuer on warps 0 / 1 (OCTIC_GEMM_ROLES_HIGH unset)                 */
+} octic_gemm_plan;
+
+int octic_gemm_last_plan(octic_gemm_plan* out);
 
 /* ---------------------------------------------------------------------------------------------------------
  * LinearD8 (octic_vits/d8_layers.py:104-127): 5 block-diagonal linears = 6 GEMM groups over packed rows.

@@ -59,6 +59,16 @@ class WgradDesc(C.Structure):
     ]
 
 
+GEMM_PLAN_TN, GEMM_PLAN_WGRAD = 0, 1
+
+
+class GemmPlan(C.Structure):
+    """Launch plan of the last GEMM on this host thread (octic_gemm_last_plan)."""
+    _fields_ = [(name, C.c_int) for name in (
+        "kind", "mode", "ncta", "num_stages", "ws", "block_n", "grid", "num_m_blocks", "total_tiles", "kb_total",
+        "full_rounds", "rem_tiles", "rem_splits", "splits", "packed", "direct", "roles_low")]
+
+
 class LsFinSeg(C.Structure):
     _fields_ = [("dw", C.c_void_p), ("w", C.c_void_p), ("N", C.c_int), ("K", C.c_int), ("gamma", C.c_void_p),
                 ("bias", C.c_void_p), ("cs", C.c_void_p), ("dgamma", C.c_void_p), ("dbias", C.c_void_p),
@@ -80,6 +90,7 @@ _P, _I, _L, _F = C.c_void_p, C.c_int, C.c_long, C.c_float
 SIGNATURES = {
     "octic_gemm_bf16": [C.POINTER(GemmDesc), _P],
     "octic_gemm_wgrad_bf16": [C.POINTER(WgradDesc), _P],
+    "octic_gemm_last_plan": [C.POINTER(GemmPlan)],
     "octic_linear_d8_pack_weights": [_P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P],
     "octic_linear_d8_fwd": [_P, _I, _I, _I, _P, _P, _P, C.POINTER(GemmDesc), _P],
     "octic_linear_d8_dgrad": [_P, _I, _I, _I, _P, _P, _P, _I, _P],

@@ -77,7 +77,7 @@ const char* octic_strerror(int code) {
   }
 }
 
-int octic_version(void) { return 200; }   // 200: round 2 (octic_attention_bwd_ws, octic_sparse_rowmap / posmap added; no entry point changed)
+int octic_version(void) { return 201; }   // 201: octic_gemm_last_plan added; 200: round 2 (octic_attention_bwd_ws, octic_sparse_rowmap / posmap added; no entry point changed)
 
 int octic_device_ok(void) {
   int dev = 0;
@@ -96,6 +96,8 @@ int octic_gemm_wgrad_bf16(const octic_wgrad_desc* desc, void* stream) {
   if (desc == nullptr || desc->dy == nullptr || desc->x == nullptr) return OCTIC_ERR_ARG;
   return launch_gemm_wgrad(desc, static_cast<cudaStream_t>(stream));
 }
+
+int octic_gemm_last_plan(octic_gemm_plan* out) { return gemm_last_plan(out); }
 
 int octic_linear_d8_pack_weights(const float* wA1, const float* wA2, const float* wB1, const float* wB2,
                                  const float* wE, int Din, int Dout, void* w1d, void* wE_packed, void* w1d_t,

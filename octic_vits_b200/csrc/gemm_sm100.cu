@@ -1227,6 +1227,17 @@ static int num_sms() {
   return g_num_sms;
 }
 
+// Plan of the last launch on this host thread (octic_gemm_last_plan): written right before the kernel launch from the
+// variables the launch uses.
+static thread_local octic_gemm_plan t_last_plan;
+static thread_local bool t_have_plan = false;
+
+int gemm_last_plan(octic_gemm_plan* out) {
+  if (out == nullptr || !t_have_plan) return OCTIC_ERR_ARG;
+  *out = t_last_plan;
+  return OCTIC_OK;
+}
+
 constexpr int kMaxDynSmem = 232448;   // 227 KiB
 // Warp-role order.  Default: TMA producer / MMA issuer on warps 0 / 1.  OCTIC_GEMM_ROLES_HIGH=1 moves them to the two
 // highest warp ids (the issue arbiter is said to prefer high warp ids); measured on B200 it is neutral to worse
@@ -1344,6 +1355,9 @@ int launch_gemm_tn(const octic_gemm_desc* d, cudaStream_t stream) {
     const octic_gemm_group& s = d->groups[i];
     GemmGroup& G = p.g[i];
     if (s.k <= 0 || s.n <= 0) return OCTIC_ERR_ARG;
+    // the A box of a group starts at column a_col: the TMA load needs it on a 16-byte boundary (a misaligned start never
+    // completes its transaction count and the pipeline's barrier wait times out)
+    if (s.a_col % 8 != 0) return OCTIC_ERR_ALIGN;
     G.a_col = s.a_col;
     G.k_blocks = (s.k + kBlockK - 1) / kBlockK;
     G.b_map = s.b_map;
@@ -1415,6 +1429,8 @@ int launch_gemm_tn(const octic_gemm_desc* d, cudaStream_t stream) {
   p.colsum = d->colsum;
   if (p.mode == EPI_GELU_BWD && (p.gelu_pre == nullptr || d->head_H > 0 || d->bias != nullptr)) return OCTIC_ERR_ARG;
   if (p.mode == EPI_RESID && p.resid_out == nullptr) return OCTIC_ERR_ARG;
+  // EPI_GELU_BF16 writes its pre-activation copy with the row stride of out: refuse a different ldb instead of ignoring it
+  if (p.mode == EPI_GELU_BF16 && p.branch_out != nullptr && d->ldb != 0 && d->ldb != d->ldo) return OCTIC_ERR_ARG;
   if (p.mode != EPI_RESID && p.out == nullptr) return OCTIC_ERR_ARG;
 
   CUtensorMap tmA, tmB0, tmB1;
@@ -1434,6 +1450,20 @@ int launch_gemm_tn(const octic_gemm_desc* d, cudaStream_t stream) {
   int grid = num_sms() / ncta;                       // CTAs (ncta = 1) or CTA pairs (ncta = 2)
   if (grid > total_tiles) grid = total_tiles;
   grid *= ncta;
+  memset(&t_last_plan, 0, sizeof(t_last_plan));
+  t_last_plan.kind = OCTIC_GEMM_PLAN_TN;
+  t_last_plan.mode = p.mode;
+  t_last_plan.ncta = ncta;
+  t_last_plan.num_stages = p.num_stages;
+  t_last_plan.ws = p.ws;
+  t_last_plan.block_n = p.block_n;
+  t_last_plan.grid = grid;
+  t_last_plan.num_m_blocks = p.num_m_blocks;
+  t_last_plan.total_tiles = total_tiles;
+  t_last_plan.packed = p.packed;
+  t_last_plan.direct = p.direct;
+  t_last_plan.roles_low = p.roles_low;
+  t_have_plan = true;
   return ncta == 2 ? launch_tn_mode<2>(p, tmA, tmB0, tmB1, grid, smem_bytes, stream)
                    : launch_tn_mode<1>(p, tmA, tmB0, tmB1, grid, smem_bytes, stream);
 }
@@ -1486,6 +1516,7 @@ int launch_gemm_wgrad(const octic_wgrad_desc* d, cudaStream_t stream) {
     const octic_wgrad_group& s = d->groups[i];
     WgradGroup& G = p.g[i];
     if (s.n_out <= 0 || s.k_in <= 0 || s.dw == nullptr) return OCTIC_ERR_ARG;
+    if (s.dy_col % 8 != 0 || s.x_col % 8 != 0) return OCTIC_ERR_ALIGN;     // TMA box starts on 16-byte boundaries
     G.dy_col = s.dy_col;
     G.x_col = s.x_col;
     G.n_out = s.n_out;
@@ -1525,6 +1556,21 @@ int launch_gemm_wgrad(const octic_wgrad_desc* d, cudaStream_t stream) {
   const SmemLayout L = smem_layout(stages, b_stage_bytes, 8);
   const int smem_bytes = L.total + 1024;
   const int grid = static_cast<int>(grid_l) * ncta;
+  memset(&t_last_plan, 0, sizeof(t_last_plan));
+  t_last_plan.kind = OCTIC_GEMM_PLAN_WGRAD;
+  t_last_plan.mode = -1;
+  t_last_plan.ncta = ncta;
+  t_last_plan.num_stages = p.num_stages;
+  t_last_plan.block_n = p.block_n;
+  t_last_plan.grid = grid;
+  t_last_plan.total_tiles = p.total_tiles;
+  t_last_plan.kb_total = kb_total;
+  t_last_plan.full_rounds = p.total_tiles / static_cast<int>(grid_l);   // the kernel's ncl = gridDim.x / NCTA
+  t_last_plan.rem_tiles = p.total_tiles - t_last_plan.full_rounds * static_cast<int>(grid_l);
+  t_last_plan.rem_splits = p.rem_splits;
+  t_last_plan.splits = p.splits;
+  t_last_plan.roles_low = p.roles_low;
+  t_have_plan = true;
   return ncta == 2 ? launch_wgrad_t<2>(p, tmDY, tmX, grid, smem_bytes, stream)
                    : launch_wgrad_t<1>(p, tmDY, tmX, grid, smem_bytes, stream);
 }

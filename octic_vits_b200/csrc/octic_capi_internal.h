@@ -52,6 +52,7 @@ struct WgradParams {
 
 int launch_gemm_tn(const octic_gemm_desc* d, cudaStream_t stream);
 int launch_gemm_wgrad(const octic_wgrad_desc* d, cudaStream_t stream);
+int gemm_last_plan(octic_gemm_plan* out);
 
 inline int roundup64(int x) { return (x + 63) / 64 * 64; }
 

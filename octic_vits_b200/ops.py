@@ -288,6 +288,14 @@ def linear_dense_wgrad(dy: torch.Tensor, x: torch.Tensor, n: int, k: int, dw: Op
     return dw
 
 
+def last_gemm_plan() -> dict:
+    """Launch plan of the last GEMM this host thread launched (see octic_gemm_plan in include/octic_b200.h), as a dict
+    of its fields.  Raises OcticError before the first GEMM launch."""
+    plan = _lib.GemmPlan()
+    _lib.check(_lib.load().octic_gemm_last_plan(C.byref(plan)), "octic_gemm_last_plan")
+    return {name: getattr(plan, name) for name, _ in plan._fields_}
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # pointwise
 # ----------------------------------------------------------------------------------------------------------------

@@ -35,10 +35,13 @@ def test_library_exports_every_header_symbol(lib):
     bound = set(_lib.SIGNATURES) | {"octic_strerror", "octic_version", "octic_device_ok",
                                       "octic_attention_headmajor_supported", "octic_attention_bwd_workspace_bytes"}
     assert set(names) == bound, set(names) ^ bound
-    assert lib.octic_version() >= 200
+    assert lib.octic_version() >= 201
     if not torch.cuda.is_available():
         # size query of the staged-dQ scratch: no device -> "the staged path does not apply" (0), never a crash
         assert lib.octic_attention_bwd_workspace_bytes(257, 80) == 0
+        # no GEMM launched on this thread yet: no launch plan to report
+        import ctypes as C
+        assert lib.octic_gemm_last_plan(C.byref(_lib.GemmPlan())) == -1
     assert lib.octic_strerror(-2).decode().startswith("pointer or leading dimension")
 
 
@@ -408,7 +411,7 @@ def test_ctypes_structs_match_the_c_header(tmp_path):
     from octic_vits_b200 import _lib
     pairs = {"octic_gemm_group": _lib.GemmGroup, "octic_gemm_desc": _lib.GemmDesc, "octic_wgrad_group": _lib.WgradGroup,
              "octic_wgrad_desc": _lib.WgradDesc, "octic_lsfin_seg": _lib.LsFinSeg, "octic_optim_chunk": _lib.OptimChunk,
-             "octic_optim_seg": _lib.OptimSeg}
+             "octic_optim_seg": _lib.OptimSeg, "octic_gemm_plan": _lib.GemmPlan}
     lines = ['#include <stdio.h>', '#include <stddef.h>', f'#include "{ROOT / "include" / "octic_b200.h"}"', 'int main(void) {']
     for cname, cls in pairs.items():
         lines.append(f'  printf("{cname} size %zu\\n", sizeof({cname}));')
