@@ -256,6 +256,15 @@ int octic_colsum_bf16(const void* x, long ldx, long T, int n_cols, float* out, v
 #define OCTIC_ATTN_DENSE 0
 #define OCTIC_ATTN_OCTIC_PACKED 1
 #define OCTIC_ATTN_OCTIC_HEADMAJOR 2
+/* 1 when the tcgen05 kernels serve the head-major layouts at (N, hd) for the given direction.  Two families do:
+ *   resident  the whole K / V (and Q / dO) of one (image, head) in one CTA's shared memory: N up to ~300 in backward
+ *             and 512 in forward;
+ *   streamed  one CTA per 128-row tile of one (image, head), the other side streamed in 64-row chunks.  Admitted only
+ *             where neither the resident kernels nor the mma.sync backward of the dense layout fit (hd 64: N > 784,
+ *             hd 80: N > 640), and for hd in {32, 64, 80, 96, 128} up to N = 8192 at least.  So every (N, hd) that
+ *             trains on the other kernels keeps its kernel; forward-only calls just below the mma.sync forward limit
+ *             (hd 64: N 785..800, hd 80: N 641..656) move here, since a layer uses one layout for both passes.
+ * Returns 0 otherwise: the packed layout (mma.sync) remains the only one there. */
 int octic_attention_headmajor_supported(int N, int hd, int backward);
 int octic_attention_fwd(const void* qkv, void* o, float* lse, int B, int N, int H, int hd, int layout,
                         void* stream);
@@ -268,7 +277,9 @@ int octic_attention_bwd(const void* qkv, const void* o, const void* d_o, const f
  * second pass that recomputes S, dP and the exponentials.  ws: octic_attention_bwd_workspace_bytes(N, hd) bytes,
  * 256-byte aligned, its first 4096 bytes zeroed once by the caller (slot flags; every launch leaves them zero); it
  * may be shared by all launches on ONE stream.  ws = NULL (or a shape the staged path does not cover: the size
- * query returns 0) runs the two-pass kernel; both produce the same gradients up to bf16 rounding of dS. */
+ * query returns 0) runs the two-pass kernel; both produce the same gradients up to bf16 rounding of dS.
+ * The streamed kernels need no workspace: dQ comes from a query-major pass that recomputes S and dP, so for their
+ * shapes (and without a device) the size query returns 0 and ws is ignored. */
 size_t octic_attention_bwd_workspace_bytes(int N, int hd);
 int octic_attention_bwd_ws(const void* qkv, const void* o, const void* d_o, const float* lse, float* delta_ws,
                            void* dqkv, int B, int N, int H, int hd, int layout, void* ws, size_t ws_bytes,

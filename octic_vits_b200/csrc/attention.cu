@@ -7,7 +7,7 @@
 // packed [T, 3D] / [T, D] rows, so the cat/permute/contiguous copies of the reference do not exist.  The dense
 // layout (deit/vit.py:36-50) is the same kernel with a trivial column map.
 //
-// One CTA per (batch, head): the whole K and V (<= 272 x 80 bf16 each) sit in shared memory; each warp owns 16 query
+// One CTA per (batch, head): the whole K and V of one (image, head) sit in shared memory; each warp owns 16 query
 // rows and runs an online-softmax loop over 64-key chunks with mma.sync.m16n8k16 (bf16 in, fp32 accumulate).
 // Backward is two passes without atomics: pass A (warps own key rows) -> dK, dV; pass B (warps own query rows) -> dQ.
 // These mma.sync kernels are the fallback for the packed-input layout and for sequences outside the envelope of the
@@ -624,6 +624,13 @@ static int make_head_map(HeadMap* m, int H, int hd, int octic) {
   return OCTIC_OK;
 }
 
+// Shared memory of the mma.sync kernels: K and V (backward pass A: Q and dO, plus lse and delta) of one (image, head).
+static bool legacy_fits(int N, int hd, bool backward) {
+  const long Npad = (N + 15) & ~15;
+  const long smem = 2 * Npad * (hd + 8) * 2 + (backward ? 2 * Npad * 4 : 0) + 3 * (hd / 2) * 4;
+  return smem <= 227 * 1024;
+}
+
 template <int HD>
 static int launch_fwd(const void* qkv, void* o, float* lse, int B, int N, int H, const HeadMap& m, cudaStream_t s) {
   const int Npad = (N + 15) & ~15;
@@ -634,7 +641,7 @@ static int launch_fwd(const void* qkv, void* o, float* lse, int B, int N, int H,
       return OCTIC_ERR_CUDA;
     done = true;
   }
-  if (smem > 227 * 1024) return OCTIC_ERR_ARG;
+  if (!legacy_fits(N, HD, false)) return OCTIC_ERR_ARG;
   const float scale_log2 = kLog2e / sqrtf(static_cast<float>(HD));
   attn_fwd_kernel<HD><<<B * H, attn_warps(N) * 32, smem, s>>>(static_cast<const __nv_bfloat16*>(qkv),
                                                               static_cast<__nv_bfloat16*>(o), lse, N, H, m, scale_log2);
@@ -654,7 +661,7 @@ static int launch_bwd(const void* qkv, const void* o, const void* d_o, const flo
       return OCTIC_ERR_CUDA;
     done = true;
   }
-  if (smem_kv > 227 * 1024) return OCTIC_ERR_ARG;
+  if (!legacy_fits(N, HD, true)) return OCTIC_ERR_ARG;
   const float scale = 1.0f / sqrtf(static_cast<float>(HD));
   const float scale_log2 = kLog2e * scale;
   launch_attn_delta(static_cast<const __nv_bfloat16*>(o), static_cast<const __nv_bfloat16*>(d_o), delta, B, N, H, m, 0, s);
@@ -669,9 +676,10 @@ static int launch_bwd(const void* qkv, const void* o, const void* d_o, const flo
 }
 
 // The tcgen05 kernels (attention_tc.cu) read head-major q, k, v (layouts OCTIC_ATTN_DENSE and
-// OCTIC_ATTN_OCTIC_HEADMAJOR) and serve every shape inside their shared-memory / TMEM envelope; the mma.sync kernels
-// above serve the packed-input octic layout and longer dense sequences.  OCTIC_ATTN_LEGACY=1 forces the latter for
-// the dense layout (A/B timing, tests).
+// OCTIC_ATTN_OCTIC_HEADMAJOR).  The resident ones serve every shape inside their shared-memory / TMEM envelope; the
+// mma.sync kernels above serve the packed-input octic layout and longer dense sequences as far as their backward fits
+// in shared memory; past that the streamed tcgen05 kernels serve the head-major layouts.  OCTIC_ATTN_LEGACY=1 forces
+// the mma.sync kernels for the dense layout (A/B timing, tests).
 static bool legacy_forced() {
   static int legacy = -1;
   if (legacy < 0) {
@@ -680,10 +688,17 @@ static bool legacy_forced() {
   }
   return legacy != 0;
 }
-static bool use_tc_path(int N, int hd, int layout, bool backward) {
-  if (layout == OCTIC_ATTN_OCTIC_PACKED) return false;
-  if (layout == OCTIC_ATTN_DENSE && legacy_forced()) return false;
-  return attn_tc_supported(N, hd, backward);
+// Streamed only where neither the resident kernels nor the mma.sync backward fit, so every shape that trains on those
+// keeps its kernel.  A layer picks one layout for both passes, hence the backward limit for forward calls too.
+static bool stream_applies(int N, int hd, bool backward) {
+  return !attn_tc_supported(N, hd, backward) && !legacy_fits(N, hd, true) && attn_stream_supported(N, hd);
+}
+enum AttnPath { kPathLegacy, kPathResident, kPathStreamed };
+static AttnPath pick_path(int N, int hd, int layout, bool backward) {
+  if (layout == OCTIC_ATTN_OCTIC_PACKED) return kPathLegacy;
+  if (layout == OCTIC_ATTN_DENSE && legacy_forced()) return kPathLegacy;
+  if (attn_tc_supported(N, hd, backward)) return kPathResident;
+  return stream_applies(N, hd, backward) ? kPathStreamed : kPathLegacy;
 }
 
 }  // namespace octic
@@ -693,7 +708,7 @@ using namespace octic;
 extern "C" {
 
 int octic_attention_headmajor_supported(int N, int hd, int backward) {
-  return attn_tc_supported(N, hd, backward != 0) ? 1 : 0;
+  return (attn_tc_supported(N, hd, backward != 0) || stream_applies(N, hd, backward != 0)) ? 1 : 0;
 }
 
 int octic_attention_fwd(const void* qkv, void* o, float* lse, int B, int N, int H, int hd, int octic_layout,
@@ -703,7 +718,9 @@ int octic_attention_fwd(const void* qkv, void* o, float* lse, int B, int N, int 
   int rc = make_head_map(&m, H, hd, octic_layout);
   if (rc) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (use_tc_path(N, hd, octic_layout, false)) return launch_attn_fwd_tc(qkv, o, lse, B, N, H, m, s);
+  const AttnPath path = pick_path(N, hd, octic_layout, false);
+  if (path == kPathResident) return launch_attn_fwd_tc(qkv, o, lse, B, N, H, m, s);
+  if (path == kPathStreamed) return launch_attn_fwd_stream(qkv, o, lse, B, N, H, m, s);
   if (octic_layout == OCTIC_ATTN_OCTIC_HEADMAJOR) return OCTIC_ERR_ARG;   // only the tcgen05 path reads this layout
   switch (hd) {
     case 32: return launch_fwd<32>(qkv, o, lse, B, N, H, m, s);
@@ -730,10 +747,12 @@ int octic_attention_bwd_ws(const void* qkv, const void* o, const void* d_o, cons
   int rc = make_head_map(&m, H, hd, octic_layout);
   if (rc) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (use_tc_path(N, hd, octic_layout, true)) {
+  const AttnPath path = pick_path(N, hd, octic_layout, true);
+  if (path != kPathLegacy) {
     launch_attn_delta(static_cast<const __nv_bfloat16*>(o), static_cast<const __nv_bfloat16*>(d_o), delta_ws, B, N, H, m,
                       octic_layout == OCTIC_ATTN_OCTIC_HEADMAJOR, s);
     if (cudaGetLastError() != cudaSuccess) return OCTIC_ERR_CUDA;
+    if (path == kPathStreamed) return launch_attn_bwd_stream(qkv, d_o, lse, delta_ws, dqkv, B, N, H, m, s);
     return launch_attn_bwd_tc(qkv, d_o, lse, delta_ws, dqkv, B, N, H, m, ws, ws_bytes, s);
   }
   if (octic_layout == OCTIC_ATTN_OCTIC_HEADMAJOR) return OCTIC_ERR_ARG;

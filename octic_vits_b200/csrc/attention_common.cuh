@@ -49,5 +49,11 @@ int launch_attn_fwd_tc(const void* qkv, void* o, float* lse, int B, int N, int H
 int launch_attn_bwd_tc(const void* qkv, const void* d_o, const float* lse, const float* delta, void* dqkv, int B, int N,
                        int H, const HeadMap& m, void* ws, size_t ws_bytes, cudaStream_t s);
 size_t attn_bwd_tc_workspace_bytes(int N, int hd);
+// streamed tcgen05 kernels (attention_tc.cu): head-major inputs of any length whose shared-memory needs fit (checked by
+// attn_stream_supported); the backward needs no workspace.  delta must already hold rowsum(dO * O).
+bool attn_stream_supported(int N, int hd);
+int launch_attn_fwd_stream(const void* qkv, void* o, float* lse, int B, int N, int H, const HeadMap& m, cudaStream_t s);
+int launch_attn_bwd_stream(const void* qkv, const void* d_o, const float* lse, const float* delta, void* dqkv, int B,
+                           int N, int H, const HeadMap& m, cudaStream_t s);
 
 }  // namespace octic

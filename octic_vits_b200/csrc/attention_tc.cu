@@ -1230,6 +1230,306 @@ __global__ void __launch_bounds__(kBwdThreads, 1) attn_bwd_tc_kernel(const __gri
 }
 
 // =====================================================================================================================
+//  streamed kernels: sequences too long for the resident kernels above
+// =====================================================================================================================
+// One CTA owns a 128-row tile of one (image, head) and streams 64-row chunks of the other side through a TMA ring, so
+// nothing in shared memory grows with N.  One template, three modes:
+//   kStreamFwd    tile = queries, chunks = K | V:   X = S = Q K^T -> P (bf16, in place) -> O += P V
+//   kStreamBwdKV  tile = keys,    chunks = Q | dO:  X = S^T = K Q^T, Y = dP^T = V dO^T -> P^T, dS^T (bf16, in place)
+//                                                   -> dV += P^T dO, dK += dS^T Q
+//   kStreamBwdQ   tile = queries, chunks = K | V:   X = S = Q K^T, Y = dP = dO V^T -> dS (bf16, in place) -> dQ += dS K
+// The backward runs the key-major and the query-major kernel one after the other: dQ is recomputed from S and dP
+// instead of reduced across key tiles, so it needs no workspace sized by B * H * N and no atomics (deterministic).
+// Warp roles: warps 0-3 do the math (thread = TMEM lane = tile row), warp 4 issues every tcgen05.mma, warp 5 every
+// chunk load.  X / Y live in two ping-pong TMEM buffers: the first-level MMAs of chunk c + 2 are issued right after the
+// second-level MMAs of chunk c (same buffer; tcgen05.mma of one thread run in issue order), while the math warps work
+// on chunk c + 1.  Operand tiles use the SWIZZLE_32B atom-column format of the resident kernels.
+enum { kStreamFwd = 0, kStreamBwdKV = 1, kStreamBwdQ = 2 };
+constexpr int kStreamCW = 64;                         // rows per streamed chunk (= TMA box rows)
+constexpr int kStreamStages = 3;
+constexpr int kStreamMath = 128;
+constexpr int kStreamThreads = kStreamMath + 64;
+
+template <int HD, int GRAN, int MODE>
+__global__ void __launch_bounds__(kStreamThreads, 1) attn_stream_tc_kernel(const __grid_constant__ CUtensorMap tmQKV,
+                                                                           const __grid_constant__ CUtensorMap tmDO,
+                                                                           __nv_bfloat16* __restrict__ out,
+                                                                           const float* __restrict__ lse_in,
+                                                                           float* __restrict__ lse_out,
+                                                                           const float* __restrict__ delta, int N, int H,
+                                                                           HeadMap m, float scale, float scale_log2) {
+  constexpr bool HAS_Y = MODE != kStreamFwd;          // second first-level product (dP / dP^T)
+  constexpr bool X_CHAIN = MODE != kStreamBwdQ;       // second level with the bf16 X as A operand (O or dV)
+  constexpr int KS = HD / 16, CW = kStreamCW, NP = CW / 16, NS = kStreamStages, NU = HD / (GRAN / 2);
+  constexpr int XS = HAS_Y ? 2 * CW : CW;             // TMEM columns of one ping-pong buffer (X, then Y)
+  constexpr int ACC = 2 * XS;                         // first accumulator column
+  constexpr int NRES = MODE == kStreamFwd ? 1 : 2;    // resident 128-row tiles
+  constexpr uint32_t kTmemCols = ACC + (MODE == kStreamBwdKV ? 2 : 1) * HD <= 256 ? 256 : 512;
+  constexpr uint32_t tile_bytes = 128 * HD * 2, chunk_bytes = CW * HD * 2;
+  enum { BAR_RES = 0, BAR_FULL = 1, BAR_EMPTY = BAR_FULL + NS, BAR_LFULL = BAR_EMPTY + NS, BAR_MDONE = BAR_LFULL + 2,
+         BAR_OFULL = BAR_MDONE + 2, BAR_ACC = BAR_OFULL + 1, NBARS = BAR_ACC + 1 };
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  const int nt = (N + 127) >> 7, nc = (N + CW - 1) / CW;
+  const int tile = blockIdx.x % nt, bh = blockIdx.x / nt, b = bh / H, h = bh - b * H, row0 = tile * 128;
+  const int npad = MODE == kStreamBwdKV ? nc * CW : 0;
+  uint8_t* A1 = smem;
+  uint8_t* A2 = A1 + (NRES - 1) * tile_bytes;
+  uint8_t* stages = A1 + NRES * tile_bytes;           // stage s: B1 chunk, then B2 chunk
+  float* lse_s = reinterpret_cast<float*>(stages + NS * 2 * chunk_bytes);   // key-major: per query column, log2 units
+  float* del_s = lse_s + npad;
+  int* cb = reinterpret_cast<int*>(del_s + npad);
+  int* sm = cb + NU;
+  uint64_t* bars = reinterpret_cast<uint64_t*>((reinterpret_cast<uintptr_t>(sm + NU) + 7) & ~uintptr_t(7));
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + NBARS);
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const long ld_out = MODE == kStreamFwd ? m.D : 3L * m.D;
+  const long soff = static_cast<long>(bh) * N;        // (b, h) row of lse / delta [B, H, N]
+
+  if (tid < NU) {
+    if (MODE == kStreamFwd) {
+      cb[tid] = o_col(m, h, tid * (GRAN / 2));
+    } else {
+      int base, smul;
+      qkv_col(m, h, tid * (GRAN / 2), base, smul);
+      cb[tid] = base; sm[tid] = smul;
+    }
+  }
+  if (MODE == kStreamBwdKV && tid < kStreamMath) {
+    for (int i = tid; i < npad; i += kStreamMath) {
+      lse_s[i] = i < N ? lse_in[soff + i] * kLog2e : INFINITY;      // +inf -> P = 0 for padded queries
+      del_s[i] = i < N ? delta[soff + i] : 0.f;
+    }
+  }
+  if (tid == kStreamMath) {
+    tma_prefetch_desc(&tmQKV);
+    tma_prefetch_desc(&tmDO);
+    mbar_init(&bars[BAR_RES], 1);
+    for (int s = 0; s < NS; ++s) { mbar_init(&bars[BAR_FULL + s], 1); mbar_init(&bars[BAR_EMPTY + s], 1); }
+    mbar_init(&bars[BAR_LFULL], 1); mbar_init(&bars[BAR_LFULL + 1], 1);
+    mbar_init(&bars[BAR_MDONE], kStreamMath); mbar_init(&bars[BAR_MDONE + 1], kStreamMath);
+    mbar_init(&bars[BAR_OFULL], 1);
+    mbar_init(&bars[BAR_ACC], 1);
+    fence_mbar_init();
+  }
+  if (warp == 4) tmem_alloc(tmem_ptr, kTmemCols);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr;
+  const uint32_t stages_addr = smem_u32(stages);
+
+  if (warp == 5) {
+    // ------------------------------------------------- load warp -------------------------------------------------
+    // head-major columns: q at h*HD, k at D + h*HD, v at 2D + h*HD of a qkv row; dO at h*HD of a dO row
+    if (lane == 0) {
+      const int colq = h * HD, colk = m.D + h * HD, colv = 2 * m.D + h * HD;
+      mbar_arrive_expect_tx(&bars[BAR_RES], NRES * tile_bytes);
+      if (MODE == kStreamBwdKV) {
+        tma_load_tile<HD>(smem_u32(A1), &tmQKV, &bars[BAR_RES], colk, row0, b, 128, CW);
+        tma_load_tile<HD>(smem_u32(A2), &tmQKV, &bars[BAR_RES], colv, row0, b, 128, CW);
+      } else {
+        tma_load_tile<HD>(smem_u32(A1), &tmQKV, &bars[BAR_RES], colq, row0, b, 128, CW);
+        if (MODE == kStreamBwdQ) tma_load_tile<HD>(smem_u32(A2), &tmDO, &bars[BAR_RES], colq, row0, b, 128, CW);
+      }
+      const CUtensorMap* mb2 = MODE == kStreamBwdKV ? &tmDO : &tmQKV;
+      const int c1 = MODE == kStreamBwdKV ? colq : colk, c2 = MODE == kStreamBwdKV ? colq : colv;
+      for (int c = 0; c < nc; ++c) {
+        const int s = c % NS;
+        if (c >= NS) mbar_wait(&bars[BAR_EMPTY + s], static_cast<uint32_t>((c / NS - 1) & 1));
+        const uint32_t dst = stages_addr + s * 2 * chunk_bytes;
+        mbar_arrive_expect_tx(&bars[BAR_FULL + s], 2 * chunk_bytes);
+        tma_load_tile<HD>(dst, &tmQKV, &bars[BAR_FULL + s], c1, c * CW, b, CW, CW);
+        tma_load_tile<HD>(dst + chunk_bytes, mb2, &bars[BAR_FULL + s], c2, c * CW, b, CW, CW);
+      }
+    }
+    __syncwarp();
+  } else if (warp == 4) {
+    // -------------------------------------------------- MMA warp --------------------------------------------------
+    const uint32_t tb = __shfl_sync(0xffffffffu, tmem_base, 0);
+    const uint32_t a1 = desc_lo_sw32(smem_u32(A1), 0), a2 = desc_lo_sw32(smem_u32(A2), 0);
+    constexpr uint32_t a_step = (128 * 32) >> 4, c_step = (CW * 32) >> 4;   // K-step = next atom column
+    const uint32_t idesc1 = make_idesc_bf16(128, CW, 0, 0), idesc2 = make_idesc_bf16(128, HD, 0, 1);
+    // first level of chunk c: X = A1 B1^T, Y = A2 B2^T (contraction over the head dim, both K-major)
+    auto issue_l1 = [&](int c) {
+      const int s = c % NS;
+      mbar_wait(&bars[BAR_FULL + s], static_cast<uint32_t>((c / NS) & 1));
+      tc_fence_after();
+      const uint32_t b1 = desc_lo_sw32(stages_addr + s * 2 * chunk_bytes, 0), b2 = b1 + (chunk_bytes >> 4);
+      const uint32_t d = tb + (c & 1) * XS;
+      if (elect_one()) {
+#pragma unroll
+        for (int ks = 0; ks < KS; ++ks) {
+          umma_ss_lohi(d, a1 + ks * a_step, b1 + ks * c_step, kDescHiSw32, idesc1, ks != 0);
+          if (HAS_Y) umma_ss_lohi(d + CW, a2 + ks * a_step, b2 + ks * c_step, kDescHiSw32, idesc1, ks != 0);
+        }
+        umma_commit(&bars[BAR_LFULL + (c & 1)]);
+      }
+      __syncwarp();
+    };
+    // second level of chunk c: acc += (bf16 X or Y in TMEM, K-step kk at column kk * 8) * chunk (MN-major, over rows)
+    auto issue_l2 = [&](int c) {
+      const int s = c % NS;
+      const uint32_t xa = tb + (c & 1) * XS, ya = xa + CW;
+      const uint32_t b1 = desc_lo_sw32(stages_addr + s * 2 * chunk_bytes, CW * 32), b2 = b1 + (chunk_bytes >> 4);
+      if (elect_one()) {
+#pragma unroll
+        for (int kk = 0; kk < NP; ++kk) {
+          const uint32_t acc = (c > 0 || kk > 0) ? 1u : 0u;
+          if (X_CHAIN)      // O += P V   or   dV += P^T dO
+            umma_ts_lohi(tb + ACC + (MODE == kStreamBwdKV ? HD : 0), xa + kk * 8, b2 + kk * 32, kDescHiSw32, idesc2, acc);
+          if (HAS_Y)        // dK += dS^T Q   or   dQ += dS K
+            umma_ts_lohi(tb + ACC, ya + kk * 8, b1 + kk * 32, kDescHiSw32, idesc2, acc);
+        }
+        umma_commit(&bars[BAR_EMPTY + s]);
+        if (MODE == kStreamFwd) umma_commit(&bars[BAR_OFULL]);
+        if (c == nc - 1) umma_commit(&bars[BAR_ACC]);
+      }
+      __syncwarp();
+    };
+    mbar_wait(&bars[BAR_RES], 0);
+    tc_fence_after();
+    issue_l1(0);
+    if (nc > 1) issue_l1(1);
+    for (int c = 0; c < nc; ++c) {
+      mbar_wait(&bars[BAR_MDONE + (c & 1)], static_cast<uint32_t>((c >> 1) & 1));
+      tc_fence_after();
+      issue_l2(c);
+      if (c + 2 < nc) issue_l1(c + 2);
+    }
+  } else {
+    // ------------------------------------------------- math warps -------------------------------------------------
+    const int rloc = tid, my_row = row0 + rloc;
+    const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(warp * 32) << 16);
+    const uint32_t lse_sa = smem_u32(lse_s), del_sa = smem_u32(del_s);
+    float lse_r = INFINITY, del_r = 0.f;                // query-major backward: this row's lse (log2 units) and delta
+    if (MODE == kStreamBwdQ && my_row < N) { lse_r = lse_in[soff + my_row] * kLog2e; del_r = delta[soff + my_row]; }
+    // forward: the row's reference maximum, raised lazily as in attn_fwd_tc_kernel (p <= 2^8 between raises)
+    const float lazy_gap = 8.0f / scale_log2;
+    float mx = -INFINITY, moff = 0.f, l = 0.f;
+    for (int c = 0; c < nc; ++c) {
+      const int buf = c & 1, k0 = c * CW;
+      mbar_wait(&bars[BAR_LFULL + buf], static_cast<uint32_t>((c >> 1) & 1));
+      tc_fence_after();
+      const uint32_t tx = t_lane + buf * XS, ty = tx + CW;
+      if (MODE == kStreamFwd) {
+        uint32_t r[NP][16];
+#pragma unroll
+        for (int q = 0; q < NP; ++q) tmem_ld_32x16(tx + q * 16, r[q]);
+        tmem_ld_wait();
+        float m0 = -INFINITY, m1 = -INFINITY;
+#pragma unroll
+        for (int q = 0; q < NP; ++q) {
+          const int nvalid = N - (k0 + q * 16);
+          if (nvalid < 16) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) r[q][i] = i < nvalid ? r[q][i] : 0xff800000u;      // -inf
+          }
+#pragma unroll
+          for (int i = 0; i < 16; i += 2) {
+            m0 = fmaxf(m0, __uint_as_float(r[q][i]));
+            m1 = fmaxf(m1, __uint_as_float(r[q][i + 1]));
+          }
+        }
+        const float mc = fmaxf(m0, m1);
+        if (c == 0) {
+          mx = mc;
+          moff = mx * scale_log2;
+        } else {
+          const bool need = mc > mx + lazy_gap;
+          if (__any_sync(0xffffffffu, need)) {
+            // O holds the P V sums of chunks < c under the old reference: wait for chunk c - 1's MMAs (chunk c's cannot
+            // have been issued), then rescale this row of O and its partial sum
+            const float f = need ? exp2f((mx - mc) * scale_log2) : 1.0f;
+            mbar_wait(&bars[BAR_OFULL], static_cast<uint32_t>((c - 1) & 1));
+            tc_fence_after();
+#pragma unroll 1
+            for (int pz = 0; pz < KS; ++pz) {
+              uint32_t ov[16];
+              tmem_ld_32x16(t_lane + ACC + pz * 16, ov);
+              tmem_ld_wait();
+              uint32_t lo[8], hi[8];
+#pragma unroll
+              for (int i = 0; i < 8; ++i) {
+                lo[i] = __float_as_uint(__uint_as_float(ov[i]) * f);
+                hi[i] = __float_as_uint(__uint_as_float(ov[8 + i]) * f);
+              }
+              tmem_st_32x8(t_lane + ACC + pz * 16, lo);
+              tmem_st_32x8(t_lane + ACC + pz * 16 + 8, hi);
+            }
+            tmem_st_wait();
+            l *= f;
+            if (need) { mx = mc; moff = mx * scale_log2; }
+          }
+        }
+        float l0 = 0.f, l1 = 0.f;
+#pragma unroll
+        for (int q = 0; q < NP; ++q) {
+          uint32_t pk[8];
+#pragma unroll
+          for (int i = 0; i < 16; i += 2) {
+            const float e0 = exp2f(fmaf(__uint_as_float(r[q][i]), scale_log2, -moff));       // -inf -> 0
+            const float e1 = exp2f(fmaf(__uint_as_float(r[q][i + 1]), scale_log2, -moff));
+            l0 += e0; l1 += e1;
+            pk[i >> 1] = pack2_bf16(e0, e1);
+          }
+          tmem_st_32x8(tx + q * 8, pk);       // bf16 P of piece q over columns of piece q / 2, already in registers
+        }
+        l += l0 + l1;
+      } else {
+        uint32_t rx[NP][16], ry[NP][16];
+#pragma unroll
+        for (int q = 0; q < NP; ++q) { tmem_ld_32x16(tx + q * 16, rx[q]); tmem_ld_32x16(ty + q * 16, ry[q]); }
+        tmem_ld_wait();
+#pragma unroll
+        for (int q = 0; q < NP; ++q) {
+          const int col0 = k0 + q * 16;
+          uint32_t pkp[8], pkd[8];
+          if (MODE == kStreamBwdKV) {
+            // columns are queries: padded ones carry lse = +inf (p = 0) and delta = 0
+            bwd_piece<true>(rx[q], ry[q], pkp, pkd, scale_log2, lse_sa + col0 * 4, del_sa + col0 * 4, 0.f, 0.f, 16);
+            tmem_st_32x8(tx + q * 8, pkp);
+          } else {
+            bwd_piece<false>(rx[q], ry[q], pkp, pkd, scale_log2, 0u, 0u, lse_r, del_r, N - col0);
+          }
+          tmem_st_32x8(ty + q * 8, pkd);
+        }
+      }
+      tmem_st_wait();
+      tc_fence_before();
+      mbar_arrive(&bars[BAR_MDONE + buf]);
+    }
+    // ---- epilogue: accumulators -> bf16 row-major staging over the resident tiles (no MMA reads them any more) ----
+    mbar_wait(&bars[BAR_ACC], 0);
+    tc_fence_after();
+    if (MODE == kStreamFwd) {
+      acc_pieces_to_stg<0, KS>(t_lane + ACC, 1.0f / l, A1 + rloc * (HD * 2));
+      if (lse_out != nullptr && my_row < N) lse_out[soff + my_row] = (mx * scale_log2 + log2f(l)) * kLn2;
+    } else {
+      acc_pieces_to_stg<0, KS>(t_lane + ACC, scale, A1 + rloc * (HD * 2));                 // dK or dQ
+      if (MODE == kStreamBwdKV) acc_pieces_to_stg<0, KS>(t_lane + ACC + HD, 1.0f, A2 + rloc * (HD * 2));   // dV
+    }
+    tc_fence_before();
+    named_bar_sync(1, kStreamMath);
+    const int nvalid = min(128, N - row0);
+    __nv_bfloat16* dst = out + (static_cast<long>(b) * N + row0) * ld_out;
+    if (MODE == kStreamFwd) {
+      store_tile<HD, GRAN>(A1, dst, ld_out, nvalid, cb, nullptr, 0, tid, kStreamMath);
+    } else {
+      store_tile<HD, GRAN>(A1, dst, ld_out, nvalid, cb, sm, MODE == kStreamBwdKV ? 1 : 0, tid, kStreamMath);
+      if (MODE == kStreamBwdKV) store_tile<HD, GRAN>(A2, dst, ld_out, nvalid, cb, sm, 2, tid, kStreamMath);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 4) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, kTmemCols);
+  }
+}
+
+// =====================================================================================================================
 //  host
 // =====================================================================================================================
 constexpr int kMaxSmem = 232448;   // 227 KiB
@@ -1414,6 +1714,72 @@ int launch_attn_bwd_tc(const void* qkv, const void* d_o, const float* lse, const
   if (!attn_tc_supported(N, m.hd, true) || !make_plan(&cp, N, m.hd)) return OCTIC_ERR_ARG;
   const int gran = pick_gran(m);
   OCTIC_TC_DISPATCH(launch_bwd_t, qkv, d_o, lse, delta, dqkv, B, N, H, m, cp, ws, ws_bytes, s)
+}
+
+
+// ---- streamed kernels ----
+static size_t stream_smem(int N, int hd, int gran, int mode) {
+  const int nu = hd / (gran / 2), nres = mode == kStreamFwd ? 1 : 2;
+  const size_t npad = mode == kStreamBwdKV ? static_cast<size_t>((N + kStreamCW - 1) / kStreamCW) * kStreamCW : 0;
+  return 1024 + static_cast<size_t>(nres * 128 + kStreamStages * 2 * kStreamCW) * hd * 2 + 2 * npad * 4 + 2 * nu * 4 + 8 +
+         (1 + 2 * kStreamStages + 6) * 8 + 16;
+}
+
+bool attn_stream_supported(int N, int hd) {
+  if (hd != 64 && hd != 80 && hd != 32 && hd != 96 && hd != 128) return false;
+  return N >= 1 && stream_smem(N, hd, 4, kStreamBwdKV) <= static_cast<size_t>(kMaxSmem);
+}
+
+template <int HD, int GRAN, int MODE>
+static int launch_stream_mode(const CUtensorMap& tmQKV, const CUtensorMap& tmDO, void* out, const float* lse_in,
+                              float* lse_out, const float* delta, int B, int N, int H, const HeadMap& m, cudaStream_t s) {
+  static bool done = false;
+  if (!done) {
+    if (cudaFuncSetAttribute(attn_stream_tc_kernel<HD, GRAN, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             kMaxSmem) != cudaSuccess)
+      return OCTIC_ERR_CUDA;
+    done = true;
+  }
+  const float scale = 1.0f / sqrtf(static_cast<float>(HD));
+  const long grid = static_cast<long>(B) * H * ((N + 127) / 128);
+  if (grid > 0x7fffffffL) return OCTIC_ERR_ARG;
+  attn_stream_tc_kernel<HD, GRAN, MODE><<<static_cast<unsigned>(grid), kStreamThreads, stream_smem(N, HD, GRAN, MODE), s>>>(
+      tmQKV, tmDO, static_cast<__nv_bfloat16*>(out), lse_in, lse_out, delta, N, H, m, scale, kLog2e * scale);
+  return cudaGetLastError() == cudaSuccess ? OCTIC_OK : OCTIC_ERR_CUDA;
+}
+
+template <int HD, int GRAN>
+static int launch_stream_fwd_t(const void* qkv, void* o, float* lse, int B, int N, int H, const HeadMap& m, cudaStream_t s) {
+  CUtensorMap tmQKV;
+  const int rc = make_map_rows(&tmQKV, qkv, B, N, 3L * m.D, kStreamCW);
+  if (rc) return rc;
+  return launch_stream_mode<HD, GRAN, kStreamFwd>(tmQKV, tmQKV, o, nullptr, lse, nullptr, B, N, H, m, s);
+}
+
+template <int HD, int GRAN>
+static int launch_stream_bwd_t(const void* qkv, const void* d_o, const float* lse, const float* delta, void* dqkv, int B,
+                               int N, int H, const HeadMap& m, cudaStream_t s) {
+  CUtensorMap tmQKV, tmDO;
+  int rc = make_map_rows(&tmQKV, qkv, B, N, 3L * m.D, kStreamCW);
+  if (rc) return rc;
+  rc = make_map_rows(&tmDO, d_o, B, N, m.D, kStreamCW);
+  if (rc) return rc;
+  rc = launch_stream_mode<HD, GRAN, kStreamBwdKV>(tmQKV, tmDO, dqkv, lse, nullptr, delta, B, N, H, m, s);
+  if (rc) return rc;
+  return launch_stream_mode<HD, GRAN, kStreamBwdQ>(tmQKV, tmDO, dqkv, lse, nullptr, delta, B, N, H, m, s);
+}
+
+int launch_attn_fwd_stream(const void* qkv, void* o, float* lse, int B, int N, int H, const HeadMap& m, cudaStream_t s) {
+  if (!attn_stream_supported(N, m.hd)) return OCTIC_ERR_ARG;
+  const int gran = pick_gran(m);
+  OCTIC_TC_DISPATCH(launch_stream_fwd_t, qkv, o, lse, B, N, H, m, s)
+}
+
+int launch_attn_bwd_stream(const void* qkv, const void* d_o, const float* lse, const float* delta, void* dqkv, int B,
+                           int N, int H, const HeadMap& m, cudaStream_t s) {
+  if (!attn_stream_supported(N, m.hd)) return OCTIC_ERR_ARG;
+  const int gran = pick_gran(m);
+  OCTIC_TC_DISPATCH(launch_stream_bwd_t, qkv, d_o, lse, delta, dqkv, B, N, H, m, s)
 }
 
 }  // namespace octic

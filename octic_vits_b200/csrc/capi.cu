@@ -77,7 +77,7 @@ const char* octic_strerror(int code) {
   }
 }
 
-int octic_version(void) { return 201; }   // 201: octic_gemm_last_plan added; 200: round 2 (octic_attention_bwd_ws, octic_sparse_rowmap / posmap added; no entry point changed)
+int octic_version(void) { return 202; }   // 202: streamed tcgen05 attention for long head-major sequences; 201: octic_gemm_last_plan added; 200: round 2 (octic_attention_bwd_ws, octic_sparse_rowmap / posmap added; no entry point changed)
 
 int octic_device_ok(void) {
   int dev = 0;
